@@ -8,8 +8,11 @@ the loop; after the loop rank 0 gathers the final latents over NCCL (configs[2])
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
   python bench.py --impl reference [--steps K] [--warmup W]      # the reference algorithm on the host CPU (oracle port)
+  python bench.py --steps K --dump-outputs DIR                    # also write the last timed step's outputs (rank 0)
 
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0). Weights and inputs are fixed by the rank's seed, so two builds run with the same arguments
+can be compared output for output: DIR/latent.npy is the latent after the last timed step ([8, 4, 32, 336], float32) and
+DIR/eps.npy that step's CFG-doubled network output ([16, 4, 32, 336], float32).
 """
 from __future__ import annotations
 
@@ -187,6 +190,7 @@ def run_reference(args) -> None:
 # ------------------------------------------------------------------------------------------------ CUDA path
 def build_pipeline(device, seed):
     from panacea_b200.pipeline import DenoisingPipeline, default_sampler_config
+    torch.manual_seed(seed)          # the default init draws on the device generator, which torch seeds at random per process
     with torch.device(device):
         pipe = DenoisingPipeline(sampler_config=default_sampler_config(50, 5.0), use_cuda_graph=True)
     pipe.model.randomize_zero_init(seed=seed)
@@ -217,6 +221,16 @@ def load_traffic():
         return d["dram_bytes_per_launch"], f"profiles/{cands[-1].name}: ncu dram__bytes_read.sum + dram__bytes_write.sum over the {d['launches']} gemm_tc launches of one eps-evaluation / launches"
     except (OSError, ValueError, KeyError):
         return None, None
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each device tensor as out_dir/<name>.npy in float32."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(d / f"{name}.npy", t.detach().float().cpu().numpy())
+    log(f"wrote {', '.join(f'{n}.npy' for n in arrays)} to {d}")
 
 
 def profile_dominant_kernel(pipe, x_in, t_dev, cc):
@@ -300,6 +314,7 @@ def run_ours(args) -> None:
         j = i % (len(sig) - 1)
         eps = wrapper(x_in, t_all[j], cc, return_static=True)
         ops.cfg_euler_step(x, eps, x_in, sig[j], sig[j + 1], 5.0, scal[j + 1][2] if j + 1 < len(scal) else scal[0][2], sigma_q=scal[j][1])
+        return eps
 
     for i in range(max(Wm, 3)):                                    # >= 3 warm-ups: packing, graph capture, clocks
         step(i)
@@ -321,9 +336,11 @@ def run_ours(args) -> None:
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for i in range(K):
-        step(i)
+        eps = step(i)
     ev1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:                            # before the e2e region overwrites x and eps
+        dump_outputs(args.dump_outputs, {"latent": x, "eps": eps})
     if dist is not None:
         dist.barrier()
     ms = ev0.elapsed_time(ev1)
@@ -425,7 +442,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's latent and eps as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -436,7 +459,8 @@ def main():
         # convenience: self-launch under torchrun when started as a plain script
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}", "--master-addr", "127.0.0.1",
                "--master-port", os.environ.get("MASTER_PORT", "29511"), str(Path(__file__).resolve()), "--gpus", str(args.gpus), "--steps",
-               str(args.steps), "--warmup", str(args.warmup)] + (["--no-cpu-baseline"] if args.no_cpu_baseline else [])
+               str(args.steps), "--warmup", str(args.warmup)] + (["--no-cpu-baseline"] if args.no_cpu_baseline else []) \
+            + (["--dump-outputs", str(Path(args.dump_outputs).resolve())] if args.dump_outputs else [])
         raise SystemExit(subprocess.call(cmd))
     run_ours(args)
 

@@ -8,6 +8,8 @@ from seeds by whoever consumes a fixture.
 from __future__ import annotations
 
 import argparse
+import gzip
+import json
 import sys
 import time
 from pathlib import Path
@@ -19,6 +21,28 @@ from . import ref_loader as R
 from . import unet_port as P
 
 GOLDEN = Path(__file__).resolve().parent.parent / "tests" / "golden"
+
+# Every fixture stays below 1 MB. Larger eps outputs are stored as the fixed sample eps.flatten()[::EPS_SAMPLE_STRIDE];
+# the stride is coprime with 2, 3 and 7, so the sample visits every frame, channel, row and column of the 32x336 and
+# 32x384 latents.
+EPS_FULL_MAX_ELEMENTS = 1 << 17
+EPS_SAMPLE_STRIDE = 5
+
+
+def shrink_eps(g: dict) -> dict:
+    """A golden_eps() record whose output is too large to store whole -> the same record with a strided sample of it
+    (`eps_shape` / `eps_stride` tell the consumer how to sample its own output the same way)."""
+    eps = g["eps"]
+    if eps.numel() <= EPS_FULL_MAX_ELEMENTS:
+        return g
+    return {**g, "eps": eps.flatten()[::EPS_SAMPLE_STRIDE].clone(), "eps_shape": tuple(eps.shape),
+            "eps_stride": EPS_SAMPLE_STRIDE}
+
+
+def trajectory_steps(num_steps: int) -> list[int]:
+    """Steps whose start-of-step latent a sampler-loop fixture keeps: the first four (the CPU port follows the first
+    three steps) and every eighth."""
+    return sorted(set(range(min(4, num_steps))) | set(range(0, num_steps, 8)))
 
 
 @torch.no_grad()
@@ -32,8 +56,25 @@ def golden_eps(case: Cs.EpsCase) -> dict:
     with R.view_height_shim(case.H, case.w):
         eps = model(x, t, dict(c))
     dt = time.time() - t0
-    return {"meta": case.meta(), "eps": eps.contiguous(), "seconds": dt, "torch": str(torch.__version__),
-            "threads": torch.get_num_threads()}
+    return shrink_eps({"meta": case.meta(), "eps": eps.contiguous(), "seconds": dt, "torch": str(torch.__version__),
+                       "threads": torch.get_num_threads()})
+
+
+@torch.no_grad()
+def golden_reference_model() -> dict:
+    """What the reference's own modules say about the network itself: the state-dict key set with shapes (tiny_3to1
+    case), the tensors its default init leaves at zero (the zero_module()'d tails), and the output of a freshly
+    constructed model on the tiny_2to1 inputs."""
+    case = Cs.GOLDEN_CASES[1]
+    sd = R.build_reference_model(case.unet_kwargs()).state_dict()
+    fresh_case = Cs.GOLDEN_CASES[0]
+    fresh = R.build_reference_model(fresh_case.unet_kwargs())
+    x, t, c = Cs.make_inputs(fresh_case)
+    out = fresh(x, t, dict(c))
+    return {"case": case.name, "state_spec": {k: list(v.shape) for k, v in sd.items()},
+            "fresh_case": fresh_case.name,
+            "fresh_zero_keys": sorted(k for k, v in fresh.state_dict().items() if not v.any()),
+            "fresh_output_shape": list(out.shape), "fresh_output_max_abs": out.abs().max().item()}
 
 
 @torch.no_grad()
@@ -93,7 +134,9 @@ def golden_sampler(case: Cs.EpsCase, num_steps: int = 10, scale: float = 5.0, us
     res = {"meta": case.meta(), "num_steps": num_steps, "scale": scale, "x_final": out, "timestep_indices": calls,
            "use_last_frame": use_last_frame, "share_noise_level": share_noise_level}
     if trajectory:
-        res["x_steps"] = torch.stack(traj)        # x as the guider sees it at the start of step i (already * sqrt(1+s0^2))
+        # x as the guider sees it at the start of step x_steps_at[k] (already * sqrt(1+s0^2))
+        res["x_steps_at"] = trajectory_steps(num_steps)
+        res["x_steps"] = torch.stack([traj[i] for i in res["x_steps_at"]])
     return res
 
 
@@ -183,6 +226,10 @@ def main(argv=None):
     if not only or "kat" in only:
         torch.save(golden_kat(), GOLDEN / "kat.pt")
         print("kat.pt")
+    if not only or "reference_model" in only:
+        with gzip.GzipFile(GOLDEN / "reference_model.json.gz", "wb", mtime=0) as f:
+            f.write(json.dumps(golden_reference_model(), indent=0).encode())
+        print("reference_model.json.gz")
     for case in Cs.GOLDEN_CASES:
         if only and case.name not in only:
             continue

@@ -1,8 +1,7 @@
 """TEST INFRASTRUCTURE — CPU oracle for the sampler loop: fp32 restatement of the reference's
 EulerEDMSampler + VanillaCFG + DiscreteDenoiser(EpsScaling, LegacyDDPMDiscretization)
 (configs/inference_nuscenes.yaml:18-28,115-126). Pinned by tests/test_oracle_golden.py against known-answer
-values computed from the reference in the build container (SURVEY.md section 8c) and, when /root/reference
-is present, against the live reference classes (tests/test_oracle_vs_reference.py).
+values and sampler loops computed from the reference in the build container (SURVEY.md section 8c).
 
 Only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs may import this module.
 """

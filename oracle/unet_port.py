@@ -6,8 +6,8 @@ module, and only as the checker / the timed CPU baseline. The product (panacea_b
 
 Pinned (not "parity unpinned"): tests/test_oracle_golden.py checks this port against golden tensors produced
 by the unmodified reference modules imported in the build container (oracle/make_golden.py, fixtures under
-tests/golden/), and tests/test_oracle_vs_reference.py re-runs the live comparison whenever /root/reference
-is present. The reference itself ships no tests or golden vectors (SURVEY.md section 4).
+tests/golden/), and tests/test_oracle_vs_reference.py checks its state-dict key set and zero-init tails against
+the reference's. The reference itself ships no tests or golden vectors (SURVEY.md section 4).
 
 It is a functional restatement, not a copy: there is no nn.Module tree, weights are looked up in a flat
 state dict by the reference's key names, the topology is derived once from the config, and the view height

@@ -78,5 +78,5 @@ def test_sampler_port_follows_the_reference_25_step_trajectory():
     x = x + c["concat"][-1].unsqueeze(0).expand_as(x) * g["share_noise_level"]
     sd, cfg = Cs.make_weights(case), case.net_config()
     out = SP.euler_edm_sample(lambda xi, ti, ci: P.wrapper_forward(sd, cfg, xi, ti, ci), x, c, uc, 25, g["scale"], max_steps=3)
-    ref = g["x_steps"][3]
+    ref = g["x_steps"][g["x_steps_at"].index(3)]
     assert ((out - ref).norm() / ref.norm()).item() < 1e-5
