@@ -8,6 +8,7 @@
  *   sgm/modules/diffusionmodules/openaimodel.py:499-542 ResBlock3D._forward
  *   sgm/modules/attention.py:407-610,229-291,1064-1134  view / text / temporal attention, STT
  *   sgm/modules/diffusionmodules/sampling.py:96-133     EulerEDMSampler step
+ *   sgm/modules/diffusionmodules/sampling.py:136-365    the other samplers' updates
  * and every entry point below names the reference call site it replaces. The Python host
  * (panacea_b200/sgm/...) mirrors those classes and binds these symbols with ctypes (INTEGRATION.md).
  *
@@ -206,6 +207,62 @@ int pn_softmax_rows(const float* in, void* out_bf16, int64_t rows, int64_t N, in
 int pn_fingerprint(const void* x, int64_t nbytes, uint64_t* out2, void* stream);
 /* out[c*n + i] = x[i] * s for c < copies (prepare_sampling_loop x *= sqrt(1+sigma0^2), CFG batch doubling). */
 int pn_scale_dup(const float* x, float* out, int64_t n, float s, int copies, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * pn_sampler_step — one fused update of the reference's samplers per network evaluation
+ * (sampling.py:96-365, sampling_utils.py:27-48, denoiser.py:22-28, guiders.py:25-29), fp32, reference operation
+ * order. Per element e < n:
+ *   den   = CFG(net2[e], net2[n+e]) with EpsScaling applied at the evaluation point xe (x, or x_eval for the *_B modes):
+ *           den_h = net_h * (-sigma_q) + xe, den = den_u + cfg_scale (den_c - den_u); net_is_denoised: den_h = net_h;
+ *   mode  PN_SAMPLER_INPUT      no network output: x only receives the noise below (EDM churn before the first step);
+ *         PN_SAMPLER_EULER      d = (x - den) / sigma; x += dt d  (EDM Euler dt = sigma_next - sigma_hat; Euler-ancestral
+ *                               dt = sigma_down - sigma; the single-evaluation steps of Heun / DPM++ 2S a);
+ *         PN_SAMPLER_HEUN_A     d = (x - den) / sigma -> d[e]; x_eval = x + dt d (x unchanged);
+ *         PN_SAMPLER_HEUN_B     d' = (x_eval - den) / sigma (sigma = sigma_next); x += ((d[e] + d') / 2) dt;
+ *         PN_SAMPLER_DPMPP2S_A  x_eval = m1 x - m2 den (x unchanged);
+ *         PN_SAMPLER_DPMPP2S_B  x = m3 x - m4 den;
+ *         PN_SAMPLER_DPMPP2M    x = m1 x - m2 (m3 den - m4 old_denoised[e]) if use_old, else x = m1 x - m2 den;
+ *                               then old_denoised[e] = den;
+ *         PN_SAMPLER_LMS        d = (x - den) / sigma -> d[lms_slot]; x += sum_j lms_coeff[j] d[(lms_slot - j) mod lms_ring]
+ *                               for j < lms_order (newest first, summed left to right);
+ *   noise (every mode but the *_A ones): x += (z * noise_mul) * noise_amp with z = noise[e] (PN_NOISE_BUFFER) or
+ *         pn_philox_normal's value for (seed, draw, e) (PN_NOISE_PHILOX);
+ *   x_in_next (optional, 2n): the next network input, (x_eval for the *_A modes, else the new x) * c_in_next, twice.
+ * d / x_eval / old_denoised are state buffers owned by the sampler (latent-sized fp32; d holds lms_ring latents for
+ * LMS); none may alias net2. */
+enum pn_sampler_mode {
+  PN_SAMPLER_INPUT = 0, PN_SAMPLER_EULER = 1, PN_SAMPLER_HEUN_A = 2, PN_SAMPLER_HEUN_B = 3,
+  PN_SAMPLER_DPMPP2S_A = 4, PN_SAMPLER_DPMPP2S_B = 5, PN_SAMPLER_DPMPP2M = 6, PN_SAMPLER_LMS = 7
+};
+enum pn_noise_source { PN_NOISE_NONE = 0, PN_NOISE_PHILOX = 1, PN_NOISE_BUFFER = 2 };
+
+typedef struct pn_sampler_args {
+  float* x;                 /* [n] latent, updated in place */
+  const float* net2;        /* [2n] network output [uncond ; cond] (NULL for PN_SAMPLER_INPUT) */
+  float* x_in_next;         /* [2n] or NULL */
+  float* x_eval;            /* [n] Heun predictor / DPM++ 2S midpoint point */
+  float* d;                 /* [n] Heun d, or [lms_ring, n] LMS derivatives */
+  float* old_denoised;      /* [n] DPM++ 2M */
+  const float* noise;       /* [n] caller-supplied N(0,1) draws (PN_NOISE_BUFFER) */
+  int64_t n;
+  uint64_t seed, draw;      /* PN_NOISE_PHILOX */
+  float sigma, sigma_q, dt;
+  float cfg_scale, c_in_next;
+  float m1, m2, m3, m4;
+  float noise_mul, noise_amp;
+  float lms_coeff[4];
+  int32_t mode;
+  int32_t net_is_denoised;
+  int32_t noise_source;
+  int32_t use_old;
+  int32_t lms_order, lms_ring, lms_slot;
+} pn_sampler_args;
+
+int pn_sampler_step(const pn_sampler_args* args, void* stream);
+/* out[e] = N(0,1) draw number `draw` of element e under `seed`: Philox4x32-10 on the counter (e / 4, draw) with key seed,
+ * Box-Muller on its two 32-bit pairs. A pure function of (seed, draw, e), independent of the launch geometry; the same
+ * values pn_sampler_step adds with PN_NOISE_PHILOX. */
+int pn_philox_normal(float* out, int64_t n, uint64_t seed, uint64_t draw, void* stream);
 
 #ifdef __cplusplus
 }

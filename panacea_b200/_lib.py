@@ -45,6 +45,19 @@ class AttnArgs(C.Structure):
     ]
 
 
+class SamplerArgs(C.Structure):
+    _fields_ = [
+        ("x", C.c_void_p), ("net2", C.c_void_p), ("x_in_next", C.c_void_p), ("x_eval", C.c_void_p), ("d", C.c_void_p),
+        ("old_denoised", C.c_void_p), ("noise", C.c_void_p),
+        ("n", C.c_int64), ("seed", C.c_uint64), ("draw", C.c_uint64),
+        ("sigma", C.c_float), ("sigma_q", C.c_float), ("dt", C.c_float), ("cfg_scale", C.c_float), ("c_in_next", C.c_float),
+        ("m1", C.c_float), ("m2", C.c_float), ("m3", C.c_float), ("m4", C.c_float),
+        ("noise_mul", C.c_float), ("noise_amp", C.c_float), ("lms_coeff", C.c_float * 4),
+        ("mode", C.c_int32), ("net_is_denoised", C.c_int32), ("noise_source", C.c_int32), ("use_old", C.c_int32),
+        ("lms_order", C.c_int32), ("lms_ring", C.c_int32), ("lms_slot", C.c_int32),
+    ]
+
+
 _vp, _i64, _i32, _f32 = C.c_void_p, C.c_int64, C.c_int32, C.c_float
 
 # name -> (restype, argtypes); every symbol declared in include/panacea_b200.h must appear here
@@ -77,6 +90,8 @@ SIGNATURES: dict[str, tuple] = {
     "pn_scale_dup": (C.c_int, [_vp, _vp, _i64, _f32, C.c_int, _vp]),
     "pn_fingerprint": (C.c_int, [_vp, _i64, _vp, _vp]),
     "pn_softmax_rows": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _f32, _vp]),
+    "pn_sampler_step": (C.c_int, [C.POINTER(SamplerArgs), _vp]),
+    "pn_philox_normal": (C.c_int, [_vp, _i64, C.c_uint64, C.c_uint64, _vp]),
 }
 
 

@@ -14,6 +14,9 @@ from . import _lib
 BF16 = torch.bfloat16
 F32 = torch.float32
 OP_BF16, OP_SPLIT3, OP_F32 = 0, 1, 2      # include/panacea_b200.h pn_operand_mode
+SAMPLER_MODES = {"input": 0, "euler": 1, "heun_a": 2, "heun_b": 3, "dpmpp2s_a": 4, "dpmpp2s_b": 5, "dpmpp2m": 6,
+                 "lms": 7}                 # include/panacea_b200.h pn_sampler_mode
+NOISE_NONE, NOISE_PHILOX, NOISE_BUFFER = 0, 1, 2   # pn_noise_source
 
 
 def _ptr(t):
@@ -395,6 +398,45 @@ class NativeOps:
                                              _stream()), "pn_cfg_euler_step")
         self.launches += 1
         return x
+
+    def sampler_step(self, mode, x, net2=None, x_in_next=None, *, x_eval=None, d=None, old_denoised=None, noise=None,
+                     seed=None, draw=0, sigma=1.0, sigma_q=None, dt=0.0, scale=1.0, c_in_next=0.0, m=(0.0, 0.0, 0.0, 0.0),
+                     noise_mul=1.0, noise_amp=0.0, lms_coeff=(), lms_ring=0, lms_slot=0, use_old=False,
+                     net_is_denoised=False):
+        """One pn_sampler_step (include/panacea_b200.h): `mode` is a key of SAMPLER_MODES. Noise: `noise` (fp32, like x)
+        adds those draws, otherwise `seed` (not None) adds the Philox draw `draw`, otherwise none is added."""
+        n = x.numel()
+        _req(x.dtype == F32 and x.is_contiguous(), "sampler_step: x must be fp32 contiguous")
+        for name, t, size in (("net2", net2, 2 * n), ("x_in_next", x_in_next, 2 * n), ("x_eval", x_eval, n),
+                              ("d", d, lms_ring * n if mode == "lms" else n), ("old_denoised", old_denoised, n), ("noise", noise, n)):
+            _req(t is None or (t.dtype == F32 and t.is_contiguous() and t.numel() == size and t.device == x.device),
+                 f"sampler_step: {name} must be fp32 contiguous with {size} elements on {x.device}")
+        a = _lib.SamplerArgs()
+        a.x, a.net2, a.x_in_next, a.x_eval, a.d, a.old_denoised, a.noise = (
+            None if t is None else t.data_ptr() for t in (x, net2, x_in_next, x_eval, d, old_denoised, noise))
+        a.n = n
+        a.noise_source = NOISE_BUFFER if noise is not None else (NOISE_PHILOX if seed is not None else NOISE_NONE)
+        a.seed, a.draw = (int(seed) if seed is not None else 0) & (2 ** 64 - 1), int(draw)
+        a.sigma, a.sigma_q, a.dt = float(sigma), float(sigma if sigma_q is None else sigma_q), float(dt)
+        a.cfg_scale, a.c_in_next = float(scale), float(c_in_next)
+        a.m1, a.m2, a.m3, a.m4 = (float(v) for v in m)
+        a.noise_mul, a.noise_amp = float(noise_mul), float(noise_amp)
+        for j, c in enumerate(lms_coeff):
+            a.lms_coeff[j] = float(c)
+        a.mode = SAMPLER_MODES[mode]
+        a.net_is_denoised, a.use_old = int(bool(net_is_denoised)), int(bool(use_old))
+        a.lms_order, a.lms_ring, a.lms_slot = len(lms_coeff), int(lms_ring), int(lms_slot)
+        _lib.check(self.lib.pn_sampler_step(C.byref(a), _stream()), "pn_sampler_step")
+        self.launches += 1
+        return x
+
+    def philox_normal(self, shape, seed, draw=0, device="cuda"):
+        """fp32 tensor of N(0,1) draws: element e is draw `draw` of e under `seed`, the values pn_sampler_step adds."""
+        out = torch.empty(shape, device=device, dtype=F32)
+        _lib.check(self.lib.pn_philox_normal(_ptr(out), out.numel(), int(seed) & (2 ** 64 - 1), int(draw), _stream()),
+                   "pn_philox_normal")
+        self.launches += 1
+        return out
 
     def softmax_rows(self, s, scale):
         """fp32 [rows, N] -> bf16 [rows, N] = softmax(scale * s) per row (VAE mid-block attention)."""
