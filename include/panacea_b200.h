@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define PN_ABI_VERSION 2
+#define PN_ABI_VERSION 3
 
 enum pn_status { PN_STATUS_OK = 0, PN_STATUS_INVALID = -1, PN_STATUS_CUDA = -2, PN_STATUS_UNSUPPORTED = -3 };
 
@@ -190,13 +190,6 @@ int pn_timestep_embedding(const int64_t* t, float* out, int64_t n, int64_t dim, 
  * (openaimodel.py:936-943, 439-445). */
 int pn_linear_small(const float* x, const void* W, int w_is_f32, const float* bias, float* y, int64_t M, int64_t N,
                     int64_t K, int64_t ldy, int silu_in, int silu_out, void* stream);
-/* One Euler step with classifier-free guidance, reference operation order (denoiser.py:22-28, guiders.py:25-29,
- * sampling_utils.py:7-9,39-40, sampling.py:103-110). net2 = [uncond ; cond] halves of n elements each: the network's
- * eps prediction (net_is_denoised = 0; the denoiser's c_out = -sigma_q, c_skip = 1 are applied here, sigma_q being
- * sigma snapped to the denoiser's 1000-entry table) or already-denoised samples (net_is_denoised = 1).
- * x is updated in place; x_in_next (optional, 2n elements) receives x_new * c_in_next duplicated. */
-int pn_cfg_euler_step(float* x, const float* net2, float* x_in_next, int64_t n, float sigma, float sigma_q,
-                      float sigma_next, float cfg_scale, float c_in_next, int net_is_denoised, void* stream);
 /* out[r, :] = softmax(scale * in[r, :]), fp32 scores -> bf16 probabilities. With two pn_gemm calls around it this is the
  * single-head attention of the VAE mid block (reference sgm/modules/diffusionmodules/model.py:374-414, head_dim = C). */
 int pn_softmax_rows(const float* in, void* out_bf16, int64_t rows, int64_t N, int64_t ld_in, int64_t ld_out, float scale,

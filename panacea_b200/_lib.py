@@ -86,7 +86,6 @@ SIGNATURES: dict[str, tuple] = {
     "pn_transpose_f32": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _i64, _vp]),
     "pn_timestep_embedding": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _vp]),
     "pn_linear_small": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp, _i64, _i64, _i64, _i64, C.c_int, C.c_int, _vp]),
-    "pn_cfg_euler_step": (C.c_int, [_vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _f32, C.c_int, _vp]),
     "pn_scale_dup": (C.c_int, [_vp, _vp, _i64, _f32, C.c_int, _vp]),
     "pn_fingerprint": (C.c_int, [_vp, _i64, _vp, _vp]),
     "pn_softmax_rows": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _f32, _vp]),

@@ -230,32 +230,7 @@ __global__ void im2col_s2_kernel(const float* __restrict__ x, void* __restrict__
   }
 }
 
-// ---------------------------------------------------------------- CFG + Euler step (sampler)
-// Follows the reference operation order in fp32 (denoiser.py:22-28 with EpsScaling c_skip=1, c_out=-sigma;
-// guiders.py:25-29 + sampling_utils.py:7-9 x_u + s (x_c - x_u); sampling_utils.py:39-40 d = (x - den)/sigma;
-// sampling.py:103-110 x += (sigma_next - sigma) d). eps holds [uncond ; cond] halves. Also emits the next
-// network input x_next * c_in(sigma_next) so the loop needs no extra pass.
-__global__ void cfg_euler_kernel(float* __restrict__ x, const float* __restrict__ net2, float* __restrict__ x_in_next,
-                                 size_t n, float sigma, float sigma_q, float sigma_next, float scale, float c_in_next,
-                                 int net_is_denoised) {
-  pdl_prologue_done();
-  for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
-    const float xv = x[e];
-    // denoiser.py:28 with EpsScaling: denoised = net * c_out + x * c_skip, c_out = -sigma_q, c_skip = 1
-    const float den_u = net_is_denoised ? net2[e] : net2[e] * (-sigma_q) + xv;
-    const float den_c = net_is_denoised ? net2[n + e] : net2[n + e] * (-sigma_q) + xv;
-    const float den = den_u + scale * (den_c - den_u);
-    const float d = (xv - den) / sigma;
-    const float xn = xv + (sigma_next - sigma) * d;
-    x[e] = xn;
-    if (x_in_next) {
-      const float v = xn * c_in_next;
-      x_in_next[e] = v;
-      x_in_next[n + e] = v;
-    }
-  }
-}
-
+// ---------------------------------------------------------------- scaled copies (sampler input, CFG batch doubling)
 __global__ void scale_dup_kernel(const float* __restrict__ x, float* __restrict__ out, size_t n, float s, int copies) {
   pdl_prologue_done();
   for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
@@ -449,16 +424,6 @@ extern "C" int pn_im2col3x3_s2(const float* x, void* out, int64_t frames, int64_
   const size_t total = (size_t)frames * Ho * Wo * 9 * (C / 8);
   PN_DISPATCH_OP(operand_mode, (launch_kernel(im2col_s2_kernel<OP>, dim3(grid_for(total)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream_v), 1, 
       x, out, (int)frames, (int)H, (int)W, (int)C, Ho, Wo, pad)));
-  PN_CHECK_CUDA(cudaGetLastError());
-  return PN_OK;
-}
-
-extern "C" int pn_cfg_euler_step(float* x, const float* net2, float* x_in_next, int64_t n, float sigma, float sigma_q,
-                                 float sigma_next, float cfg_scale, float c_in_next, int net_is_denoised,
-                                 void* stream_v) {
-  PN_REQUIRE(x && net2 && n > 0 && sigma > 0.f, "pn_cfg_euler_step: bad arguments");
-  launch_kernel(cfg_euler_kernel, dim3(grid_for((size_t)n)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream_v), 1, 
-      x, net2, x_in_next, (size_t)n, sigma, sigma_q, sigma_next, cfg_scale, c_in_next, net_is_denoised);
   PN_CHECK_CUDA(cudaGetLastError());
   return PN_OK;
 }

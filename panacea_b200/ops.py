@@ -390,14 +390,11 @@ class NativeOps:
         return y
 
     def cfg_euler_step(self, x, net2, x_in_next, sigma, sigma_next, scale, c_in_next, sigma_q=None, net_is_denoised=False):
-        _req(x.dtype == F32 and net2.dtype == F32 and x.is_contiguous() and net2.is_contiguous() and net2.numel() == 2 * x.numel(),
-             "cfg_euler_step: shapes")
-        sq = sigma if sigma_q is None else sigma_q
-        _lib.check(self.lib.pn_cfg_euler_step(_ptr(x), _ptr(net2), _ptr(x_in_next), x.numel(), float(sigma), float(sq),
-                                             float(sigma_next), float(scale), float(c_in_next), int(bool(net_is_denoised)),
-                                             _stream()), "pn_cfg_euler_step")
-        self.launches += 1
-        return x
+        """One CFG + Euler step from sigma to sigma_next: the "euler" mode of sampler_step. dt is the float32 difference
+        of the float32-rounded sigmas, like the reference's tensors (a float64 difference can differ in the last bit)."""
+        from .sgm.modules.diffusionmodules.sampling_utils import sub32      # not at the top: sgm imports this module
+        return self.sampler_step("euler", x, net2, x_in_next, sigma=sigma, sigma_q=sigma_q, dt=sub32(sigma_next, sigma),
+                                 scale=scale, c_in_next=c_in_next, net_is_denoised=net_is_denoised)
 
     def sampler_step(self, mode, x, net2=None, x_in_next=None, *, x_eval=None, d=None, old_denoised=None, noise=None,
                      seed=None, draw=0, sigma=1.0, sigma_q=None, dt=0.0, scale=1.0, c_in_next=0.0, m=(0.0, 0.0, 0.0, 0.0),

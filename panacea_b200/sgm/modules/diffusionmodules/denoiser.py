@@ -2,7 +2,7 @@
 
 Host side: the ascending 1000-entry sigma table, sigma<->index snapping (`sigma_to_idx` = nearest table entry)
 and the per-step scalars. Device side: `input * c_in` and `net * c_out + input * c_skip` are fused into
-pn_scale_dup / pn_cfg_euler_step by the sampler; `__call__` below keeps the reference call signature for
+pn_sampler_step by the sampler; `__call__` below keeps the reference call signature for
 callers that use the denoiser on its own (one elementwise kernel per call)."""
 from __future__ import annotations
 

@@ -1,5 +1,5 @@
 """guiders.py:8-40 VanillaCFG: batch doubling (unconditional half first) and x_u + scale (x_c - x_u).
-The combine itself runs inside the fused sampler kernel (pn_cfg_euler_step); this class carries the scale and
+The combine itself runs inside the fused sampler kernel (pn_sampler_step); this class carries the scale and
 builds the doubled conditioning ONCE per sample instead of once per step."""
 from __future__ import annotations
 

@@ -1,15 +1,12 @@
 """sampling.py:24-365: the reference's samplers around one fused update kernel per network evaluation.
 
-EulerEDMSampler with s_churn = 0 — "DDIM (eta=0)" in the reference config (configs/inference_nuscenes.yaml:115-126) —
-runs one eps evaluation of the CFG-doubled batch (ControlNet + UNet, optionally one CUDA graph replay) and ONE fused
-kernel (pn_cfg_euler_step) per step that applies the denoiser scalings, the guidance combination, the Euler update and
-the next step's input scaling + batch doubling. The reference's per-step torch.cat / dict rebuild (guiders.py:31-40)
-happens once per sample here.
-
-The other samplers (EDM Euler with churn, Heun, Euler-ancestral, DPM++ 2S a, DPM++ 2M, LMS) follow the same pattern
-with pn_sampler_step: their sigma-dependent scalars are computed on the host once per sample (sampling_utils.py, the
-reference's float32 expressions), and every network evaluation is followed by exactly one kernel that applies the
-denoiser scalings, the guidance, the sampler's update, its noise and writes the next network input. State that a
+Every sampler — EulerEDMSampler (with s_churn = 0 the "DDIM (eta=0)" of the reference config,
+configs/inference_nuscenes.yaml:115-126, or with churn), Heun, Euler-ancestral, DPM++ 2S a, DPM++ 2M, LMS — runs
+through the one host loop of `_Sampler`: the sigma-dependent scalars are computed on the host once per sample
+(sampling_utils.py, the reference's float32 expressions), and every eps evaluation of the CFG-doubled batch (ControlNet
++ UNet, optionally one CUDA graph replay) is followed by exactly one pn_sampler_step that applies the denoiser
+scalings, the guidance, the sampler's update, its noise and writes the next network input (scaled and batch-doubled).
+The reference's per-step torch.cat / dict rebuild (guiders.py:31-40) happens once per sample here. State that a
 sampler keeps between evaluations (Heun's d, the evaluation point of Heun / DPM++ 2S, DPM++ 2M's old denoised, LMS's
 derivatives) lives in latent-sized fp32 buffers the sampler owns, never in the network's output buffer.
 
@@ -21,7 +18,6 @@ discards), and before every EDM step with gamma > 0 (the reference's torch.randn
 and must return N(0,1) draws of its shape."""
 from __future__ import annotations
 
-import math
 from dataclasses import dataclass, field
 
 import torch
@@ -35,7 +31,7 @@ DEFAULT_GUIDER = {"target": "sgm.modules.diffusionmodules.guiders.IdentityGuider
 class BoundDenoiser:
     """What `DiffusionEngine3D.sample` passes to the sampler in the reference is a lambda closing over
     (denoiser, model) (diffusion.py:251-254); this object is the same callable with the two parts visible, so the
-    sampler can fuse the denoiser scalings, the guidance and the Euler update into one kernel per step."""
+    sampler can fuse the denoiser scalings, the guidance and its update into one kernel per evaluation."""
 
     def __init__(self, denoiser, network):
         self.denoiser = denoiser
@@ -227,50 +223,8 @@ class EDMSampler(_Sampler):
 
 
 class EulerEDMSampler(EDMSampler):
-    """sampling.py:214-218. s_churn = 0 (the reference config) runs the single pn_cfg_euler_step per step below."""
-
-    @torch.no_grad()
-    def __call__(self, denoiser, x, cond, uc=None, num_steps=None):
-        if self.s_churn != 0.0:
-            return super().__call__(denoiser, x, cond, uc, num_steps)
-        ops = self.ops
-        uc = default(uc, cond)
-        sig = [float(s) for s in self.sigmas(num_steps)]
-        self._check_guider()
-        n = x.shape[0]
-        # prepare_sampling_loop (sampling.py:44-55): x *= sqrt(1 + sigma_0^2)
-        x = ops.scale_dup(x.float().contiguous(), math.sqrt(1.0 + sig[0] ** 2.0), 1)
-        if not isinstance(denoiser, BoundDenoiser):
-            return self._euler_generic_loop(ops, denoiser, x, cond, uc, sig)
-        den, net = denoiser.denoiser, denoiser.network
-        cc = self.guider.prepare_cond(cond, uc)                   # once per sample
-        if hasattr(net, "prepare"):
-            net.prepare(cc)                                       # step-invariant conditioning work, once per sample
-        scal = [den.step_scalars(s) for s in sig[:-1]]
-        self.last_timestep_indices = [s[0] for s in scal]
-        t_all = torch.tensor([[s[0]] * (2 * n) for s in scal], dtype=torch.int64, device=x.device)
-        x_in = ops.scale_dup(x, scal[0][2], 2)                    # input * c_in, CFG batch doubling
-        for i in range(len(sig) - 1):
-            eps = net(x_in, t_all[i], cc, return_static=True) if hasattr(net, "static_io") else net(x_in, t_all[i], cc)
-            c_in_next = scal[i + 1][2] if i + 1 < len(scal) else 0.0
-            ops.cfg_euler_step(x, eps, x_in, sig[i], sig[i + 1], self.guider.scale, c_in_next, sigma_q=scal[i][1])
-            if self.step_callback is not None:
-                self.step_callback(i, x)
-        return x
-
-    def _euler_generic_loop(self, ops, denoiser, x, cond, uc, sig):
-        """The reference's call contract (sampling.py:85-133): an opaque `denoiser(x2, sigma2, cond2) -> denoised2` per
-        step with the guider's doubled inputs; guidance combination + Euler update in one kernel (net_is_denoised)."""
-        n = x.shape[0]
-        self.last_timestep_indices = []
-        for i in range(len(sig) - 1):
-            s_in = torch.full((n,), sig[i], dtype=torch.float32, device=x.device)
-            x2, s2, c2 = self.guider.prepare_inputs(x, s_in, cond, uc)
-            den2 = denoiser(x2, s2, c2).float().contiguous()
-            ops.cfg_euler_step(x, den2, None, sig[i], sig[i + 1], self.guider.scale, 0.0, net_is_denoised=True)
-            if self.step_callback is not None:
-                self.step_callback(i, x)
-        return x
+    """sampling.py:214-218. With s_churn = 0 (the reference config) every step is one "euler" evaluation at
+    sigma_hat = sigma, with no noise."""
 
 
 class HeunEDMSampler(EDMSampler):

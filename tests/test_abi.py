@@ -28,13 +28,15 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, n), f"{n} declared in the header but not exported"
         assert n in _lib.SIGNATURES, f"{n} has no ctypes signature"
     assert set(_lib.SIGNATURES) == set(names)
-    assert lib.pn_abi_version() == 2
+    assert lib.pn_abi_version() == 3
 
 
 def test_struct_layout_matches_header_field_order():
     from panacea_b200 import _lib
+    from panacea_b200.ops import SAMPLER_MODES
     text = (ROOT / "include" / "panacea_b200.h").read_text()
-    for cname, cls in (("pn_gemm_args", _lib.GemmArgs), ("pn_attn_args", _lib.AttnArgs)):
+    for cname, cls in (("pn_gemm_args", _lib.GemmArgs), ("pn_attn_args", _lib.AttnArgs),
+                       ("pn_sampler_args", _lib.SamplerArgs)):
         body = re.search(r"typedef struct %s \{(.*?)\} %s;" % (cname, cname), text, flags=re.S).group(1)
         body = re.sub(r"/\*.*?\*/", "", body, flags=re.S)
         fields = []
@@ -45,6 +47,8 @@ def test_struct_layout_matches_header_field_order():
             for part in decl.split(","):
                 fields.append(re.sub(r"\[.*?\]", "", part.strip().split()[-1].lstrip("*")))
         assert fields == [f[0] for f in cls._fields_], (cname, fields)
+    modes = dict(re.findall(r"PN_SAMPLER_([A-Z0-9_]+) = (\d+)", text))
+    assert {k.lower(): int(v) for k, v in modes.items()} == SAMPLER_MODES
 
 
 def test_compute_entry_points_fail_loudly_without_cuda():

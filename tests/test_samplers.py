@@ -1,8 +1,7 @@
-"""CPU tests of the reference's other samplers (sampling.py:136-365): host scalars against known-answer values of the
-unmodified reference (tests/golden/sampler_family_kat.pt, python -m oracle.sampler_family), the C struct of
-pn_sampler_step, and the samplers' host loops run through a torch restatement of the kernel modes (TorchSamplerOps
-below) against the reference's own trajectories."""
-import re
+"""CPU tests of the reference's samplers (sampling.py:85-365): host scalars against known-answer values of the
+unmodified reference (tests/golden/sampler_family_kat.pt, python -m oracle.sampler_family), and the samplers' host
+loops run through a torch restatement of the kernel modes (TorchRefOps.sampler_step) against the reference's own
+trajectories."""
 from pathlib import Path
 
 import pytest
@@ -14,64 +13,8 @@ from oracle import sampler_port as SP
 from oracle import unet_port as P
 from torch_ref_ops import TorchRefOps
 
-ROOT = Path(__file__).resolve().parent.parent
 GOLDEN = Path(__file__).resolve().parent / "golden"
 F32 = torch.float32
-
-
-class TorchSamplerOps(TorchRefOps):
-    """pn_sampler_step restated with fp32 torch tensor ops in the reference's operation order
-    (include/panacea_b200.h). Noise comes from the caller's buffer only: the in-kernel Philox is not restated here."""
-
-    def sampler_step(self, mode, x, net2=None, x_in_next=None, *, x_eval=None, d=None, old_denoised=None, noise=None,
-                     seed=None, draw=0, sigma=1.0, sigma_q=None, dt=0.0, scale=1.0, c_in_next=0.0, m=(0.0, 0.0, 0.0, 0.0),
-                     noise_mul=1.0, noise_amp=0.0, lms_coeff=(), lms_ring=0, lms_slot=0, use_old=False,
-                     net_is_denoised=False):
-        self.launches += 1
-        n = x.shape[0]
-        m1, m2, m3, m4 = m
-        new_x, next_in = x, None
-        if mode != "input":
-            xe = x_eval if mode in ("heun_b", "dpmpp2s_b") else x
-            du, dc = net2[:n], net2[n:]
-            if not net_is_denoised:
-                sq = sigma if sigma_q is None else sigma_q
-                du, dc = du * -sq + xe, dc * -sq + xe
-            den = du + scale * (dc - du)
-        if mode == "euler":
-            new_x = x + dt * ((x - den) / sigma)
-        elif mode == "heun_a":
-            dd = (x - den) / sigma
-            d.copy_(dd)
-            next_in = x + dt * dd
-            x_eval.copy_(next_in)
-        elif mode == "heun_b":
-            new_x = x + ((d + (x_eval - den) / sigma) / 2.0) * dt
-        elif mode == "dpmpp2s_a":
-            next_in = m1 * x - m2 * den
-            x_eval.copy_(next_in)
-        elif mode == "dpmpp2s_b":
-            new_x = m3 * x - m4 * den
-        elif mode == "dpmpp2m":
-            new_x = m1 * x - m2 * ((m3 * den - m4 * old_denoised) if use_old else den)
-            old_denoised.copy_(den)
-        elif mode == "lms":
-            ring = d.view(lms_ring, *x.shape)
-            ring[lms_slot] = (x - den) / sigma
-            acc = 0
-            for j, c in enumerate(lms_coeff):
-                acc = acc + c * ring[(lms_slot - j) % lms_ring]
-            new_x = x + acc
-        if next_in is None:
-            if seed is not None:
-                raise NotImplementedError("in-kernel Philox noise is not restated on the CPU")
-            if noise is not None:
-                new_x = new_x + noise * noise_mul * noise_amp
-            x.copy_(new_x)
-            next_in = x
-        if x_in_next is not None:
-            x_in_next.copy_(torch.cat([next_in, next_in]) * c_in_next)
-        return x
 
 
 @pytest.fixture(scope="module")
@@ -120,24 +63,6 @@ def test_lms_coefficients_are_the_exact_integrals(kat):
         U.linear_multistep_coeff(3, t64, 1, 0)
 
 
-def test_sampler_args_struct_matches_header_field_order():
-    from panacea_b200 import _lib
-    text = (ROOT / "include" / "panacea_b200.h").read_text()
-    body = re.search(r"typedef struct pn_sampler_args \{(.*?)\} pn_sampler_args;", text, flags=re.S).group(1)
-    body = re.sub(r"/\*.*?\*/", "", body, flags=re.S)
-    fields = []
-    for decl in body.split(";"):
-        decl = decl.strip()
-        if not decl:
-            continue
-        for part in decl.split(","):
-            fields.append(re.sub(r"\[.*?\]", "", part.strip().split()[-1].lstrip("*")))
-    assert fields == [f[0] for f in _lib.SamplerArgs._fields_], fields
-    from panacea_b200.ops import SAMPLER_MODES
-    modes = dict(re.findall(r"PN_SAMPLER_([A-Z0-9_]+) = (\d+)", text))
-    assert {k.lower(): int(v) for k, v in modes.items()} == SAMPLER_MODES
-
-
 def test_reference_targets_instantiate():
     from panacea_b200.sgm.util import instantiate_from_config
     for name, (cls, kw) in MG.SAMPLER_FAMILY.items():
@@ -165,7 +90,7 @@ def _run(name, disc, network, x, c, uc, fused):
     from panacea_b200.pipeline import DEFAULT_DENOISER
     from panacea_b200.sgm.modules.diffusionmodules.sampling import BoundDenoiser
     from panacea_b200.sgm.util import instantiate_from_config
-    ops = TorchSamplerOps()
+    ops = TorchRefOps()
     sampler = _make(name, disc, ops)
     noise = MG.SeededNoise()
     sampler.noise_sampler = noise
@@ -212,10 +137,10 @@ def test_ancestral_eta_zero_is_the_euler_sampler():
     x, c, uc = MG.closed_form_inputs()
     port = SP.DiscreteDenoiserPort()
     den = lambda xx, s, cc: port(MG.closed_form_network, xx, s, cc)        # noqa: E731
-    ea = _make("euler_ancestral", ops=TorchSamplerOps())
+    ea = _make("euler_ancestral", ops=TorchRefOps())
     ea.eta = 0.0
     ea.noise_sampler = lambda z: pytest.fail("noise drawn at eta = 0")
-    eu = _make("euler_churn", ops=TorchSamplerOps())
+    eu = _make("euler_churn", ops=TorchRefOps())
     eu.s_churn = 0.0                # the reference config's Euler sampler
     a = ea(den, x.clone(), c, uc)
     b = SP.euler_edm_sample(MG.closed_form_network, x.clone(), c, uc, MG.FAMILY_STEPS, MG.FAMILY_SCALE)

@@ -10,7 +10,7 @@ import torch
 
 from oracle import cases as Cs
 from oracle import sampler_family as MG
-from test_samplers import TorchSamplerOps
+from torch_ref_ops import TorchRefOps
 
 pytestmark = pytest.mark.gpu
 
@@ -65,7 +65,7 @@ def test_sampler_step_mode_vs_torch(ops, mode, net_is_denoised):
     state = {"x_eval": r(*LATENT), "d": r(kw.get("lms_ring", 1) * n0, *LATENT[1:]), "old_denoised": r(*LATENT)}
     noise = r(*LATENT) if "noise_amp" in kw else None
     outs = []
-    for o in (ops, TorchSamplerOps()):
+    for o in (ops, TorchRefOps()):
         xx, st = x.clone(), {k: v.clone() for k, v in state.items()}
         xin = torch.zeros(2 * n0, *LATENT[1:], device="cuda")
         o.sampler_step(mode, xx, None if mode == "input" else net2, xin, sigma_q=2.9, scale=5.0, c_in_next=0.33,
@@ -194,8 +194,8 @@ def _bf16_gain(name):
 
 
 def test_equivalences_and_default_noise():
-    """EulerAncestralSampler(eta=0) is EulerEDMSampler; the in-kernel noise follows torch.manual_seed; the plain-callable
-    path agrees with the fused path."""
+    """EulerAncestralSampler(eta=0) is EulerEDMSampler (the default sampler, with its launch count); the in-kernel noise
+    follows torch.manual_seed; the plain-callable path agrees with the fused path."""
     from panacea_b200.pipeline import default_sampler_config
     from panacea_b200.sgm.modules.diffusionmodules.sampling import BoundDenoiser
     from panacea_b200.sgm.util import instantiate_from_config
@@ -205,7 +205,10 @@ def test_equivalences_and_default_noise():
     ea = _make("euler_ancestral")
     ea.eta = 0.0
     eu = instantiate_from_config(default_sampler_config(MG.FAMILY_STEPS, MG.FAMILY_SCALE))
-    assert _rel(ea(fn, x.clone(), c, uc), eu(fn, x.clone(), c, uc)) <= 1e-6
+    launches = eu.ops.launches
+    x_eu = eu(fn, x.clone(), c, uc)
+    assert eu.ops.launches - launches == 2 + MG.FAMILY_STEPS          # scale, first input, one per evaluation
+    assert _rel(ea(fn, x.clone(), c, uc), x_eu) <= 1e-6
     runs = []
     for name in ("euler_ancestral", "heun_churn"):
         s = _make(name)

@@ -200,15 +200,56 @@ class TorchRefOps:
         y = F.linear(F.silu(x) if silu_in else x, w.float(), bias)
         return F.silu(y) if silu_out else y
 
-    def cfg_euler_step(self, x, net2, x_in_next, sigma, sigma_next, scale, c_in_next, sigma_q=None, net_is_denoised=False):
+    def sampler_step(self, mode, x, net2=None, x_in_next=None, *, x_eval=None, d=None, old_denoised=None, noise=None,
+                     seed=None, draw=0, sigma=1.0, sigma_q=None, dt=0.0, scale=1.0, c_in_next=0.0, m=(0.0, 0.0, 0.0, 0.0),
+                     noise_mul=1.0, noise_amp=0.0, lms_coeff=(), lms_ring=0, lms_slot=0, use_old=False,
+                     net_is_denoised=False):
+        """pn_sampler_step restated with fp32 torch tensor ops in the reference's operation order
+        (include/panacea_b200.h). Noise comes from the caller's buffer only: the in-kernel Philox is not restated here."""
+        self.launches += 1
         n = x.shape[0]
-        sq = sigma if sigma_q is None else sigma_q
-        den_u = net2[:n] if net_is_denoised else net2[:n] * (-sq) + x
-        den_c = net2[n:] if net_is_denoised else net2[n:] * (-sq) + x
-        den = den_u + scale * (den_c - den_u)
-        x.copy_(x + (sigma_next - sigma) * ((x - den) / sigma))
+        m1, m2, m3, m4 = m
+        new_x, next_in = x, None
+        if mode != "input":
+            xe = x_eval if mode in ("heun_b", "dpmpp2s_b") else x
+            du, dc = net2[:n], net2[n:]
+            if not net_is_denoised:
+                sq = sigma if sigma_q is None else sigma_q
+                du, dc = du * -sq + xe, dc * -sq + xe
+            den = du + scale * (dc - du)
+        if mode == "euler":
+            new_x = x + dt * ((x - den) / sigma)
+        elif mode == "heun_a":
+            dd = (x - den) / sigma
+            d.copy_(dd)
+            next_in = x + dt * dd
+            x_eval.copy_(next_in)
+        elif mode == "heun_b":
+            new_x = x + ((d + (x_eval - den) / sigma) / 2.0) * dt
+        elif mode == "dpmpp2s_a":
+            next_in = m1 * x - m2 * den
+            x_eval.copy_(next_in)
+        elif mode == "dpmpp2s_b":
+            new_x = m3 * x - m4 * den
+        elif mode == "dpmpp2m":
+            new_x = m1 * x - m2 * ((m3 * den - m4 * old_denoised) if use_old else den)
+            old_denoised.copy_(den)
+        elif mode == "lms":
+            ring = d.view(lms_ring, *x.shape)
+            ring[lms_slot] = (x - den) / sigma
+            acc = 0
+            for j, c in enumerate(lms_coeff):
+                acc = acc + c * ring[(lms_slot - j) % lms_ring]
+            new_x = x + acc
+        if next_in is None:
+            if seed is not None:
+                raise NotImplementedError("in-kernel Philox noise is not restated on the CPU")
+            if noise is not None:
+                new_x = new_x + noise * noise_mul * noise_amp
+            x.copy_(new_x)
+            next_in = x
         if x_in_next is not None:
-            x_in_next.copy_(torch.cat([x, x]) * c_in_next)
+            x_in_next.copy_(torch.cat([next_in, next_in]) * c_in_next)
         return x
 
     def scale_dup(self, x, s, copies):

@@ -102,7 +102,7 @@ def main(argv=None):
         upd = [st_.elapsed_time(en_) * 1e3 for st_, en_ in timed.events]
         rec = {"sampler": name, "class": cls, "kwargs": kw, "steps": a.steps, "evaluations_per_sample": evals,
                "update_kernels": len(upd) // a.repeats,
-               "update_us_per_evaluation": sum(upd) / max(len(upd), 1) if cls != "EulerEDMSampler" or kw else None,
+               "update_us_per_evaluation": sum(upd) / max(len(upd), 1),
                "ms_per_sample": min(times), "ms_per_sample_all": times, "ms_per_evaluation": min(times) / evals,
                "latent": list(noise.shape), "cfg_scale": 5.0, "precision": "bf16", "gpu": info}
         print(json.dumps(rec), flush=True)
